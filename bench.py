@@ -8,6 +8,7 @@ parameter blocks, one worker per GPU, batch 128 per worker, synthetic CIFAR10, r
     python bench.py --impl reference --gpus N ...            # the unmodified reference through an offline shim
     python bench.py --driver consensus --bb ...              # BASELINE config 3 (adaptive ADMM); --driver fedprox
                                                              # --optimizer lbfgs (config 4); --driver vae | cpc (config 5)
+    python bench.py ... --dump-outputs DIR                   # also save what the last step computed (see dump_outputs)
 
 A *step* is one minibatch optimizer step on every worker (128*N images): zero-grad, forward, CE loss, backward,
 fused Adam on the active block, and the reference's post-step diagnostics forward; block aggregation (fused
@@ -52,6 +53,25 @@ PRIME_STEPS = 4           # eager warm-up + CUDA-graph capture of the step, befo
 # The device window straddles the SECOND round boundary: the first aggregation of a run is warm-up like the first minibatches are
 # (first cross-GPU touch of the block's peer-mapped pages; on one 8-GPU box it cost 9 ms once, the next ones 0.7 ms — r2_scaling.md).
 TIMED_BOUNDARY = 2 * STEPS_PER_ROUND
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, eng) -> None:
+    """Write what a caller of the training step receives once the run's last step is done: that step's loss
+    (``loss.npy``) and the trained model, every ``state_dict`` entry of replica 0 as ``<model>.<key>.npy`` in its logical
+    shape.  Inputs (synthetic data, initialisation) are seeded, so two builds run with the same arguments can be compared
+    file for file."""
+    import numpy as np
+
+    arrays = {"loss": eng.last_loss1.detach().float().reshape(1)}
+    for model, net in eng.replicas[0].nets.items():
+        for key, t in net.state_dict().items():
+            arrays["%s.%s" % (model, key)] = t.detach().float() if t.is_floating_point() else t.detach().double()
+    total = sum(t.numel() * t.element_size() for t in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs of %d bytes exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().contiguous().numpy())
 
 
 # ----------------------------------------------------------------------------------------------
@@ -330,6 +350,8 @@ def run_ours(args) -> dict:
 
     eng.step_hook = hook
     eng.run()
+    if args.dump_outputs and topo.is_root:
+        dump_outputs(args.dump_outputs, eng)
     ms_d = _max_over_ranks(ev_d[0].elapsed_time(ev_d[1]), dev)
     images = 128 * N * K
     value = images / (ms_d / 1e3)
@@ -406,13 +428,19 @@ def main():
     ap.add_argument("--no-fast", dest="no_fast", action="store_true")
     ap.add_argument("--no-e2e", dest="no_e2e", action="store_true")
     ap.add_argument("--no-collective-table", dest="no_collective_table", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss and the trained model to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.algo == "admm":
         args.driver = "consensus"
     if args.impl == "nccl":   # the "baseline, not the product": stock ATen ops, eager, NCCL all-reduce on the flat block
         args.no_fast, args.no_graphs, args.collective = True, True, "torch"
 
+    if args.dump_outputs and (args.impl == "reference" or args.driver in ("vae", "vae_cl", "cpc")):
+        ap.error("--dump-outputs is supported for the ResNet18 drivers (federated, consensus, fedprox) of this implementation")
     if args.impl == "reference":
         from baseline.ref_shim import run_reference_bench
 

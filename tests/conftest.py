@@ -1,43 +1,12 @@
-import importlib.util
 import os
 import sys
-
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
-
-REFERENCE_SRC = "/root/reference/src"
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
     config.addinivalue_line("markers", "multigpu: needs >= 2 CUDA devices")
 
-
-def _load_reference(name):
-    """Import a module of the reference under a private name (oracle only; never product code)."""
-    path = os.path.join(REFERENCE_SRC, name + ".py")
-    if not os.path.exists(path):
-        pytest.skip("reference not mounted")
-    spec = importlib.util.spec_from_file_location("_ref_" + name, path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
-@pytest.fixture(scope="session")
-def ref_models():
-    return _load_reference("simple_models")
-
-
-@pytest.fixture(scope="session")
-def ref_lbfgs():
-    return _load_reference("lbfgsnew")
-
-
-@pytest.fixture(scope="session")
-def ref_utils():
-    # simple_utils imports torchvision at module import; fine here
-    return _load_reference("simple_utils")

@@ -3,6 +3,8 @@ import os
 
 import torch
 
+import golden_data
+
 from federated_pytorch_test_b200 import models
 from federated_pytorch_test_b200.config import (CPCConfig, ConsensusConfig, FedProxConfig, FederatedConfig,
                                                 NoConsensusConfig, VAECLConfig, parse_config)
@@ -30,22 +32,32 @@ def test_cli_overrides():
     assert c.use_resnet is False and c.Nloop == 2
 
 
-def test_legacy_checkpoint_interop(tmp_path, ref_models):
-    net = models.Net()
+def test_legacy_checkpoint_interop(tmp_path):
+    g = golden_data.load("test_models")          # the reference's Net: state_dict layout, output with seeded weights
+    layout = dict(zip(g["Net/keys"], g["Net/shapes"]))
+    net = golden_data.fill_(models.Net())
     FlatArena(net)
     opt = torch.optim.Adam(net.parameters())
     path = ckpt.save_worker(str(tmp_path), 3, net, 0, opt, 1.25)
     assert os.path.basename(path) == "s3.model"
     blob = torch.load(path, weights_only=False)
     assert sorted(blob) == ["epoch", "model_state_dict", "optimizer_state_dict", "running_loss"]
-    ref = ref_models.Net()
-    ref.load_state_dict(blob["model_state_dict"])          # the reference can read our file
-    x = torch.randn(2, 3, 32, 32)
-    torch.testing.assert_close(ref(x), net(x))
-    torch.save({"model_state_dict": ref_models.Net().state_dict(), "epoch": 0, "optimizer_state_dict": {}, "running_loss": 0.0},
+    # the reference can read our file: its strict load_state_dict needs these keys and shapes, and the values it
+    # loads are the seeded weights, on which it computes the stored output
+    sd = blob["model_state_dict"]
+    assert {k: ",".join(map(str, v.shape)) for k, v in sd.items()} == layout
+    seeded = golden_data.fill_(models.Net()).state_dict()
+    for k, v in sd.items():
+        assert torch.equal(v, seeded[k]), k
+    golden_data.assert_matches(net(golden_data.randn(4, 3, 32, 32, seed=1)), g, "Net/out")
+    gen = torch.Generator().manual_seed(5)
+    ref_sd = {k: torch.randn(*(int(d) for d in shape.split(",") if d), generator=gen) for k, shape in layout.items()}
+    torch.save({"model_state_dict": ref_sd, "epoch": 0, "optimizer_state_dict": {}, "running_loss": 0.0},
                ckpt.worker_path(str(tmp_path), 4))
     ckpt.load_worker(str(tmp_path), 4, net, "cpu")          # and we can read the reference's
     assert net._flat_arena.check_views() and net.training
+    for k, v in net.state_dict().items():
+        assert torch.equal(v, ref_sd[k]), k
 
 
 def test_log_formats_golden():

@@ -3,10 +3,13 @@ block visit against a literal reference-style loop, multi-process (gloo) == sing
 import os
 import sys
 
+import numpy as np
 import pytest
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
+
+import golden_data
 
 from federated_pytorch_test_b200 import models
 from federated_pytorch_test_b200.api import (consensus_multi, federated_cpc, federated_multi, federated_vae,
@@ -106,20 +109,21 @@ def test_vae_vaecl_cpc_drivers(tmp_path):
 
 
 # ----------------------------------------------------------------------------------------------
-def test_block_visit_matches_reference_style_loop(ref_utils, ref_models):
-    """One ADMM block visit: BlockAdam + closed-form penalty on arena slices  ==  the reference recipe
-    (torch.optim.Adam + autograd through torch.cat, get/put_trainable_values) on the same batches."""
-    from federated_pytorch_test_b200.algo.engine import Engine, EngineConfig, Replica, Task, Visit
-    from federated_pytorch_test_b200.algo.strategies import ADMM
-    from federated_pytorch_test_b200.parallel import Topology, TorchCollective
-    from federated_pytorch_test_b200.utils import init_weights
+K_VISIT, B_VISIT, STEPS_VISIT, ROUNDS_VISIT, RHO_VISIT, CI_VISIT, LAM1_VISIT, LAM2_VISIT = 2, 16, 3, 2, 0.1, 4, 1e-4, 1e-4
 
-    K, B, steps, rounds, rho, ci = 2, 16, 3, 2, 0.1, 4
+
+def _visit_data():
     g = torch.Generator().manual_seed(0)
-    data = {k: [(torch.randn(B, 3, 32, 32, generator=g), torch.randint(0, 10, (B,), generator=g)) for _ in range(steps)] for k in range(K)}
-    lam1, lam2 = 1e-4, 1e-4
+    return {k: [(torch.randn(B_VISIT, 3, 32, 32, generator=g), torch.randint(0, 10, (B_VISIT,), generator=g))
+                for _ in range(STEPS_VISIT)] for k in range(K_VISIT)}
 
-    # ---- reference-style ----
+
+def golden(ref):
+    """The reference recipe of one ADMM block visit (torch.optim.Adam + autograd through torch.cat,
+    get/put_trainable_values) on the reference's Net and utilities; see golden_data.py."""
+    ref_models, ref_utils = ref.models, ref.utils
+    K, steps, rounds, rho, ci, lam1, lam2 = K_VISIT, STEPS_VISIT, ROUNDS_VISIT, RHO_VISIT, CI_VISIT, LAM1_VISIT, LAM2_VISIT
+    data = _visit_data()
     nets = {}
     for k in range(K):
         nets[k] = ref_models.Net()
@@ -151,8 +155,25 @@ def test_block_visit_matches_reference_style_loop(ref_utils, ref_models):
             primal += float(torch.norm(yd))
             ys[k].add_(yd)
         ref_trace.append((primal / N, dual))
+    out = {"visit/trace": np.array(ref_trace)}
+    for k in range(K):
+        out.update(golden_data.digest(ref_utils.get_trainable_values(nets[k]), "visit/x%d" % k))
+    return out
 
-    # ---- engine ----
+
+def test_block_visit_matches_reference_style_loop():
+    """One ADMM block visit: BlockAdam + closed-form penalty on arena slices  ==  the reference recipe (``golden``
+    above) on the same batches."""
+    from federated_pytorch_test_b200.algo.engine import Engine, EngineConfig, Replica, Task, Visit
+    from federated_pytorch_test_b200.algo.strategies import ADMM
+    from federated_pytorch_test_b200.parallel import Topology, TorchCollective
+    from federated_pytorch_test_b200.utils import init_weights
+
+    K, rounds, rho, ci, lam1, lam2 = K_VISIT, ROUNDS_VISIT, RHO_VISIT, CI_VISIT, LAM1_VISIT, LAM2_VISIT
+    data = _visit_data()
+    g = golden_data.load("test_engine")
+    ref_trace = [tuple(r) for r in g["visit/trace"]]
+
     class FixedTask(Task):
         def build_replica(self, ck, device, allocator):
             net = models.Net()
@@ -180,12 +201,13 @@ def test_block_visit_matches_reference_style_loop(ref_utils, ref_models):
     strat = ADMM(coll, topo, 5, rho0=rho)
     eng = Engine(FixedTask(), topo, strat, coll, EngineConfig(Nloop=1, Nadmm=rounds, Nepoch=1), log=lambda m: None)
     eng.run()
+    assert len(trace) == len(ref_trace) == rounds
     for (p1, d1), (p2, d2) in zip(ref_trace, trace):
         assert p2 == pytest.approx(p1, rel=2e-3) and d2 == pytest.approx(d1, rel=2e-3)
     lo, hi = models.Net().train_order_block_ids()[ci]
     for k in range(K):
         mine = eng.replicas[k].arenas["net"].compact(lo, hi)
-        torch.testing.assert_close(mine, ref_utils.get_trainable_values(nets[k]), rtol=1e-3, atol=1e-5)
+        golden_data.assert_matches(mine, g, "visit/x%d" % k, rtol=1e-3, atol=1e-5)
 
 
 # ----------------------------------------------------------------------------------------------

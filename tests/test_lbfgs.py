@@ -1,10 +1,12 @@
 """LBFGSNew against the reference implementation (SURVEY §2.5, §4)."""
 import warnings
 
-import pytest
+import numpy as np
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
+
+import golden_data
 
 from federated_pytorch_test_b200.optim import LBFGSNew
 from federated_pytorch_test_b200.utils import FlatArena
@@ -37,12 +39,24 @@ def test_rosenbrock_golden():
     assert (calls, iters) == (655, 31)  # BASELINE.md §2
 
 
-def test_rosenbrock_identical_to_reference(ref_lbfgs):
-    a, b = _rosenbrock(ref_lbfgs.LBFGSNew), _rosenbrock(LBFGSNew)
-    assert torch.equal(a[0], b[0]) and a[1:] == b[1:]
+def test_rosenbrock_identical_to_reference():
+    g = golden_data.load("test_lbfgs")
+    x, *counts = _rosenbrock(LBFGSNew)
+    assert torch.equal(x, torch.from_numpy(g["rosenbrock/x"])) and counts == g["rosenbrock/counts"].tolist()
 
 
 def _stochastic(cls, arena=False, steps=5):
+    """Five stochastic L-BFGS steps on one CPU thread: the iterates are compared bit for bit with stored values, and
+    the convolution's weight gradient is a reduction whose rounding depends on how many threads share it."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        return _stochastic_run(cls, arena, steps)
+    finally:
+        torch.set_num_threads(threads)
+
+
+def _stochastic_run(cls, arena, steps):
     torch.manual_seed(0)
     net = nn.Sequential(nn.Conv2d(3, 8, 3), nn.ELU(), nn.Flatten(), nn.Linear(8 * 30 * 30, 10))
     if arena:
@@ -70,18 +84,28 @@ def _stochastic(cls, arena=False, steps=5):
     return log, vec, opt
 
 
-def test_stochastic_identical_to_reference(ref_lbfgs):
-    a, b = _stochastic(ref_lbfgs.LBFGSNew), _stochastic(LBFGSNew)
-    assert [x[1:] for x in a[0]] == [x[1:] for x in b[0]]          # forward/backward counts per step
-    assert torch.equal(a[1], b[1])                                 # bit-identical iterates
-    ka = sorted(a[2].state_dict()["state"][0].keys())
-    kb = sorted(b[2].state_dict()["state"][0].keys())
-    assert ka == kb
+def golden(ref):
+    """The reference's LBFGSNew on the two problems above; see golden_data.py."""
+    x, *counts = _rosenbrock(ref.lbfgs.LBFGSNew)
+    log, vec, opt = _stochastic(ref.lbfgs.LBFGSNew)
+    return {"rosenbrock/x": x.numpy(), "rosenbrock/counts": np.array(counts),
+            "stochastic/counts": np.array([x[1:] for x in log]), "stochastic/sha256": np.array(golden_data.sha256(vec)),
+            "stochastic/state_keys": np.array(sorted(opt.state_dict()["state"][0].keys()))}
 
 
-def test_stochastic_on_arena_close_to_reference(ref_lbfgs):
-    a, c = _stochastic(ref_lbfgs.LBFGSNew), _stochastic(LBFGSNew, arena=True)
-    assert [x[1:] for x in a[0]] == [x[1:] for x in c[0]]
+def test_stochastic_identical_to_reference():
+    g = golden_data.load("test_lbfgs")
+    log, vec, opt = _stochastic(LBFGSNew)
+    assert [list(x[1:]) for x in log] == g["stochastic/counts"].tolist()       # forward/backward counts per step
+    assert golden_data.sha256(vec) == str(g["stochastic/sha256"])             # bit-identical iterates
+    assert sorted(opt.state_dict()["state"][0].keys()) == list(g["stochastic/state_keys"])
+
+
+def test_stochastic_on_arena_close_to_reference():
+    g = golden_data.load("test_lbfgs")
+    a, c = _stochastic(LBFGSNew), _stochastic(LBFGSNew, arena=True)
+    assert golden_data.sha256(a[1]) == str(g["stochastic/sha256"])            # a is the reference's result, bit for bit
+    assert [list(x[1:]) for x in c[0]] == g["stochastic/counts"].tolist()
     torch.testing.assert_close(a[1], c[1], rtol=1e-4, atol=1e-5)
     assert c[2]._v().fused
 

@@ -1,6 +1,9 @@
 """Model zoo: shapes, parameter/block inventory (SURVEY §2.2) and forward parity with the reference."""
+import numpy as np
 import pytest
 import torch
+
+import golden_data
 
 from federated_pytorch_test_b200 import models
 from federated_pytorch_test_b200.ops import functional as FX
@@ -47,67 +50,118 @@ PAIRS = [("Net", lambda m: m.Net(), (4, 3, 32, 32)), ("Net1", lambda m: m.Net1()
          ("ContextgenCNN", lambda m: m.ContextgenCNN(32), (2, 32, 3, 3))]
 
 
-@pytest.mark.parametrize("name,make,shape", PAIRS)
-def test_forward_matches_reference(ref_models, name, make, shape):
-    """Same state_dict keys, and identical outputs when given the reference's weights."""
+def _layout(name, net):
+    sd = net.state_dict()
+    return {name + "/keys": np.array(list(sd)), name + "/shapes": np.array([",".join(map(str, t.shape)) for t in sd.values()])}
+
+
+def _forward(m, make, shape):
+    """``make(m)`` with the seeded weights of ``golden_data.fill_`` and its output on a seeded input."""
     FX.set_fast_path(False)
-    torch.manual_seed(0)
-    ref = make(ref_models)
-    mine = make(models)
-    assert list(ref.state_dict().keys()) == list(mine.state_dict().keys())
-    mine.load_state_dict(ref.state_dict())
-    x = torch.randn(*shape)
-    torch.testing.assert_close(mine(x), ref(x), rtol=1e-5, atol=1e-5)
+    net = golden_data.fill_(make(m))
+    return net, net(golden_data.randn(*shape, seed=1))
 
 
-def test_encoder_predictor_match_reference(ref_models):
-    torch.manual_seed(0)
-    ref, mine = ref_models.EncoderCNN(64), models.EncoderCNN(64)
-    mine.load_state_dict(ref.state_dict())
-    x = torch.randn(6, 8, 32, 32)
-    torch.testing.assert_close(mine(x), ref(x), rtol=1e-5, atol=1e-5)
-    rp, mp = ref_models.PredictorCNN(64, 8), models.PredictorCNN(64, 8)
-    mp.load_state_dict(rp.state_dict())
-    a, b = torch.randn(2, 64, 3, 3), torch.randn(2, 64, 3, 3)
-    for u, v in zip(mp(a, b), rp(a, b)):
-        torch.testing.assert_close(u, v)
+def _encoder_predictor(m):
+    enc = golden_data.fill_(m.EncoderCNN(64), seed=2)
+    pred = golden_data.fill_(m.PredictorCNN(64, 8), seed=3)
+    y = enc(golden_data.randn(6, 8, 32, 32, seed=4))
+    return enc, pred, [y] + list(pred(golden_data.randn(2, 64, 3, 3, seed=5), golden_data.randn(2, 64, 3, 3, seed=6)))
 
 
-def test_vae_deterministic_parts_match_reference(ref_models):
-    torch.manual_seed(0)
-    ref, mine = ref_models.AutoEncoderCNN(), models.AutoEncoderCNN()
-    mine.load_state_dict(ref.state_dict())
-    x = torch.rand(3, 3, 32, 32)
-    for u, v in zip(mine.encode(x), ref.encode(x)):
-        torch.testing.assert_close(u, v, rtol=1e-5, atol=1e-6)
-    z = torch.randn(3, 10)
-    torch.testing.assert_close(mine.decode(z), ref.decode(z), rtol=1e-5, atol=1e-6)
+def _uniform(*shape, seed):
+    return torch.rand(*shape, generator=torch.Generator().manual_seed(seed))
 
 
-def test_vae_cl_batched_equals_loop(ref_models):
-    torch.manual_seed(0)
-    ref = ref_models.AutoEncoderCNNCL(K=4, L=8)
-    a = models.AutoEncoderCNNCL(K=4, L=8, batched_clusters=True)
-    b = models.AutoEncoderCNNCL(K=4, L=8, batched_clusters=False)
-    a.load_state_dict(ref.state_dict())
-    b.load_state_dict(ref.state_dict())
+def _vae(m):
+    net = golden_data.fill_(m.AutoEncoderCNN(), seed=7)
+    return net, list(net.encode(_uniform(3, 3, 32, 32, seed=8))) + [net.decode(golden_data.randn(3, 10, seed=9))]
+
+
+_EK = torch.zeros(5, 4)
+_EK[:, 2] = 1
+
+
+def _vae_cl_heads(net):
+    """encodeclus, then the deterministic heads of cluster 2 (encode, decode)."""
+    x = _uniform(5, 3, 32, 32, seed=11)
+    return [net.encodeclus(x)], list(net.encode(x, _EK)), list(net.decode(_EK, golden_data.randn(5, 8, seed=12)))
+
+
+def golden(ref):
+    """What the reference computes in the comparisons below (see golden_data.py)."""
+    out = {}
+    for name, make, shape in PAIRS:
+        net, y = _forward(ref.models, make, shape)
+        out.update(_layout(name, net), **golden_data.digest(y, name + "/out"))
+    enc, pred, ys = _encoder_predictor(ref.models)
+    out.update(_layout("EncoderCNN", enc), **_layout("PredictorCNN", pred))
+    for i, y in enumerate(ys):
+        out.update(golden_data.digest(y, "encoder_predictor/%d" % i))
+    net, ys = _vae(ref.models)
+    out.update(_layout("AutoEncoderCNN", net))
+    for i, y in enumerate(ys):
+        out.update(golden_data.digest(y, "vae/%d" % i))
+    net = golden_data.fill_(ref.models.AutoEncoderCNNCL(K=4, L=8), seed=10)
+    out.update(_layout("AutoEncoderCNNCL", net))
+    for part, ys in zip(("encodeclus", "encode", "decode"), _vae_cl_heads(net)):
+        for i, y in enumerate(ys):
+            out.update(golden_data.digest(y, "vae_cl/%s/%d" % (part, i)))
+    return out
+
+
+def _check_layout(name, net):
+    g = golden_data.load("test_models")
+    mine = _layout(name, net)
+    assert list(mine[name + "/keys"]) == list(g[name + "/keys"]) and list(mine[name + "/shapes"]) == list(g[name + "/shapes"])
+
+
+@pytest.mark.parametrize("name,make,shape", PAIRS)
+def test_forward_matches_reference(name, make, shape):
+    """Same state_dict layout as the reference, and the reference's outputs when given the same weights."""
+    net, y = _forward(models, make, shape)
+    _check_layout(name, net)
+    golden_data.assert_matches(y, golden_data.load("test_models"), name + "/out", rtol=1e-5, atol=1e-5)
+
+
+def test_encoder_predictor_match_reference():
+    enc, pred, ys = _encoder_predictor(models)
+    _check_layout("EncoderCNN", enc)
+    _check_layout("PredictorCNN", pred)
+    g = golden_data.load("test_models")
+    assert len([k for k in g if k.startswith("encoder_predictor/") and k.endswith("/shape")]) == len(ys)
+    golden_data.assert_matches(ys[0], g, "encoder_predictor/0", rtol=1e-5, atol=1e-5)
+    for i, y in enumerate(ys[1:], 1):
+        golden_data.assert_matches(y, g, "encoder_predictor/%d" % i)
+
+
+def test_vae_deterministic_parts_match_reference():
+    net, ys = _vae(models)
+    _check_layout("AutoEncoderCNN", net)
+    g = golden_data.load("test_models")
+    assert len([k for k in g if k.startswith("vae/") and k.endswith("/shape")]) == len(ys)
+    for i, y in enumerate(ys):
+        golden_data.assert_matches(y, g, "vae/%d" % i, rtol=1e-5, atol=1e-6)
+
+
+def test_vae_cl_batched_equals_loop():
+    a = golden_data.fill_(models.AutoEncoderCNNCL(K=4, L=8, batched_clusters=True), seed=10)
+    b = golden_data.fill_(models.AutoEncoderCNNCL(K=4, L=8, batched_clusters=False), seed=10)
+    _check_layout("AutoEncoderCNNCL", a)
     a.force_disable_repr()
     b.force_disable_repr()
-    x = torch.rand(5, 3, 32, 32)
-    torch.testing.assert_close(a.encodeclus(x), ref.encodeclus(x), rtol=1e-5, atol=1e-6)
+    # encodeclus and the deterministic heads against the reference, cluster by cluster
+    g = golden_data.load("test_models")
+    for part, ys in zip(("encodeclus", "encode", "decode"), _vae_cl_heads(a)):
+        assert len([k for k in g if k.startswith("vae_cl/%s/" % part) and k.endswith("/shape")]) == len(ys)
+        for i, y in enumerate(ys):
+            golden_data.assert_matches(y, g, "vae_cl/%s/%d" % (part, i), rtol=1e-5, atol=1e-6)
+    x = _uniform(5, 3, 32, 32, seed=11)
     oa, ob = a(x), b(x)
     torch.testing.assert_close(oa[0], ob[0])
     for da, db in zip(oa[1:], ob[1:]):
         for k in range(4):
             torch.testing.assert_close(da[k], db[k], rtol=1e-5, atol=1e-6)
-    # deterministic heads against the reference, cluster by cluster
-    ek = torch.zeros(5, 4)
-    ek[:, 2] = 1
-    for u, v in zip(a.encode(x, ek), ref.encode(x, ek)):
-        torch.testing.assert_close(u, v, rtol=1e-5, atol=1e-6)
-    z = torch.randn(5, 8)
-    for u, v in zip(a.decode(ek, z), ref.decode(ek, z)):
-        torch.testing.assert_close(u, v, rtol=1e-5, atol=1e-6)
 
 
 def test_disable_repr_quirk_preserved():

@@ -3,7 +3,9 @@ rounds), the TF32-rounding fp64 oracle, the benchmark's window placement and the
 import importlib.util
 import math
 import os
+import types
 
+import numpy as np
 import pytest
 import torch
 import torch.nn as nn
@@ -94,10 +96,15 @@ def test_tf32_rounding_and_oracle():
     assert errs[-1] < 1e-2                                        # last bias: sum of dy, rounded only through dy's dependence
 
 
-def test_bench_windows_straddle_the_second_and_a_later_boundary():
+def _bench():
     spec = importlib.util.spec_from_file_location("_bench_mod", os.path.join(ROOT, "bench.py"))
     b = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(b)
+    return b
+
+
+def test_bench_windows_straddle_the_second_and_a_later_boundary():
+    b = _bench()
     spr = b.STEPS_PER_ROUND
     assert b.TIMED_BOUNDARY == 2 * spr
     for K, W in ((20, 5), (40, 5), (10, 3), (2, 3), (100, 5), (200, 10)):
@@ -111,6 +118,22 @@ def test_bench_windows_straddle_the_second_and_a_later_boundary():
         fe = b.straddle_window(K, W, b_host, b_host + spr)
         assert fe >= b_host + min(W, spr) or K >= 2 * spr
         assert fe <= b_host + spr - 1 and fe + K >= b_host + spr + 1
+
+
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs: the last step's loss and every state_dict entry of the trained model, float32 / float64 .npy."""
+    torch.manual_seed(0)
+    net = nn.Sequential(nn.Conv2d(3, 4, 3), nn.BatchNorm2d(4))
+    net(torch.randn(2, 3, 8, 8))
+    eng = types.SimpleNamespace(last_loss1=torch.tensor(0.25), replicas=[types.SimpleNamespace(nets={"net": net})])
+    _bench().dump_outputs(str(tmp_path), eng)
+    sd = net.state_dict()
+    assert sorted(os.listdir(tmp_path)) == sorted(["loss.npy"] + ["net.%s.npy" % k for k in sd])
+    assert np.load(tmp_path / "loss.npy").tolist() == [0.25]
+    for k, v in sd.items():
+        a = np.load(tmp_path / ("net.%s.npy" % k))
+        assert a.dtype in (np.float32, np.float64) and a.shape == tuple(v.shape)
+        assert np.array_equal(a, v.double().numpy())
 
 
 def test_dilated_stem_and_tiny_map_conv_cpu_fallback():

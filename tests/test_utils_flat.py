@@ -1,7 +1,10 @@
 """simple_utils API + flat arena (SURVEY §2.3, §4 unit level)."""
+import numpy as np
 import pytest
 import torch
 import torch.nn as nn
+
+import golden_data
 
 from federated_pytorch_test_b200 import models
 from federated_pytorch_test_b200.utils import (FlatArena, freeze_all_layers, get_trainable_values, init_weights,
@@ -39,26 +42,51 @@ def test_block_masks_and_roundtrip(factory, use_arena):
     assert [p.requires_grad for p in net.parameters()][:3] == [True, True, False][: min(3, n)]
 
 
-def test_pack_matches_reference(ref_utils, ref_models):
-    torch.manual_seed(1)
-    ref, mine = ref_models.Net(), models.Net()
-    mine.load_state_dict(ref.state_dict())
-    FlatArena(mine)
+def _packed(m, unfreeze, get_values, arena=False):
+    """get_trainable_values of every block of Net (seeded weights), block after block."""
+    net = golden_data.fill_(m.Net(), seed=13)
+    if arena:
+        FlatArena(net)
+    out = []
     for b in range(5):
-        ref_utils.unfreeze_one_block(ref, b)
-        unfreeze_one_block(mine, b)
-        torch.testing.assert_close(get_trainable_values(mine), ref_utils.get_trainable_values(ref))
+        unfreeze(net, b)
+        out.append(get_values(net))
+    return out
 
 
-def test_init_weights_matches_reference(ref_utils, ref_models):
-    ref, mine = ref_models.ResNet9(), models.ResNet9()
-    FlatArena(mine, channels_last_weights=True)   # values must not depend on the memory format
+def _initialised(m, init, arena=False):
+    net = m.ResNet9()
+    if arena:
+        FlatArena(net, channels_last_weights=True)   # values must not depend on the memory format
     torch.manual_seed(0)
-    ref.apply(ref_utils.init_weights)
-    torch.manual_seed(0)
-    mine.apply(init_weights)
-    for (k, a), (_, b) in zip(mine.state_dict().items(), ref.state_dict().items()):
-        torch.testing.assert_close(a.contiguous(), b, msg=k)
+    net.apply(init)
+    return net
+
+
+def golden(ref):
+    """What the reference computes in the comparisons below (see golden_data.py)."""
+    out = {}
+    for b, v in enumerate(_packed(ref.models, ref.utils.unfreeze_one_block, ref.utils.get_trainable_values)):
+        out.update(golden_data.digest(v, "pack/%d" % b))
+    sd = _initialised(ref.models, ref.utils.init_weights).state_dict()
+    out["init/keys"] = np.array(list(sd))
+    for k, v in sd.items():
+        out.update(golden_data.digest(v, "init/" + k, k=64))
+    return out
+
+
+def test_pack_matches_reference():
+    g = golden_data.load("test_utils_flat")
+    for b, v in enumerate(_packed(models, unfreeze_one_block, get_trainable_values, arena=True)):
+        golden_data.assert_matches(v, g, "pack/%d" % b)
+
+
+def test_init_weights_matches_reference():
+    g = golden_data.load("test_utils_flat")
+    sd = _initialised(models, init_weights, arena=True).state_dict()
+    assert list(sd) == list(g["init/keys"])
+    for k, a in sd.items():
+        golden_data.assert_matches(a.contiguous(), g, "init/" + k)
     # ConvTranspose2d untouched (Q15): default init differs from xavier, bias not 0.01
     vae = models.AutoEncoderCNN()
     vae.apply(init_weights)
